@@ -1,9 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- the driver's measurement contract for the VisionLLMv2 forward hot path.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--dump-outputs DIR]
 
 One JSON line on rank 0.  See DESIGN.md "Measurement" for what each field means.
+With --dump-outputs, rank 0 also writes the arrays its last timed step returned to DIR/<name>.npy (see dump_outputs),
+so that two builds can be compared output for output on the same seeded inputs.  It needs --impl native: the reference
+arm times a bounded CPU sample of the path (one layer per tower), not the path's outputs.
 Workloads live in bench_workloads.py; the default is the most complete
 native path available (see DEFAULT_WORKLOAD there).
 """
@@ -76,6 +79,58 @@ def trace(msg):
         print(f"[bench rank {os.environ.get('RANK', '0')} +{time.time() - _T0:6.1f}s] {msg}", file=sys.stderr, flush=True)
 
 
+DUMP_BUDGET_BYTES = 64 * 10 ** 6
+NPY_HEADER_BYTES = 128                     # numpy writes a 128-byte header for these 1-D / few-dim arrays
+
+
+def dump_outputs(out, directory, budget=DUMP_BUDGET_BYTES):
+    """Write every tensor in one step's result (nested dicts / lists / tuples, e.g. a ModelOutput) as
+    `directory/<dotted name>.npy`: floating types other than float64 become float32; float64 and integer types become
+    float64 (exact for integers below 2^53).  When that would take more than `budget` bytes, each array is replaced by
+    a sample of its flattened elements -- distinct indices drawn by a generator seeded with 0, sorted, a share of the
+    budget proportional to the array's size, at least one element -- and the indices are written as float64 to
+    `directory/sample_index/<dotted name>.npy`.  The budget counts whole files, headers included.  The same elements are written on every run
+    with the same arguments.  Returns {name: {"shape", "dtype", "elements_written"}}."""
+    import numpy as np
+    import torch
+    arrays = {}
+
+    def walk(name, x):
+        if isinstance(x, torch.Tensor):
+            arrays[name or "out"] = x.detach()
+        elif isinstance(x, dict):
+            for k, v in x.items():
+                walk(f"{name}.{k}" if name else str(k), v)
+        elif isinstance(x, (list, tuple)):
+            for i, v in enumerate(x):
+                walk(f"{name}.{i}" if name else str(i), v)
+
+    walk("", out)
+    if not arrays:
+        raise RuntimeError(f"--dump-outputs: the step returned no tensors ({type(out).__name__})")
+    wide = {n: t.dtype == torch.float64 or not (t.is_floating_point() or t.dtype == torch.bool) for n, t in arrays.items()}
+    width = {n: 8 if wide[n] else 4 for n in arrays}
+    sampled = sum(t.numel() * width[n] + NPY_HEADER_BYTES for n, t in arrays.items()) > budget
+    if sampled:
+        cost = sum(t.numel() * (width[n] + 8) for n, t in arrays.items())     # value + float64 index per element
+        room = budget - (16 + 2 * NPY_HEADER_BYTES) * len(arrays)            # headers, at-least-one-element guarantee
+        os.makedirs(os.path.join(directory, "sample_index"), exist_ok=True)
+    os.makedirs(directory, exist_ok=True)
+    manifest = {}
+    for name, t in arrays.items():
+        flat = t.reshape(-1)
+        if sampled and flat.numel():
+            keep = min(flat.numel(), max(1, flat.numel() * room // cost))
+            g = torch.Generator(device=flat.device).manual_seed(0)
+            idx = torch.randperm(flat.numel(), generator=g, device=flat.device)[:keep].sort().values
+            flat = flat[idx]
+            np.save(os.path.join(directory, "sample_index", name + ".npy"), idx.to(torch.float64).cpu().numpy())
+        a = flat.to(torch.float64 if wide[name] else torch.float32).cpu().numpy()
+        np.save(os.path.join(directory, name + ".npy"), a if sampled else a.reshape(tuple(t.shape)))
+        manifest[name] = {"shape": list(t.shape), "dtype": str(t.dtype).replace("torch.", ""), "elements_written": a.size}
+    return manifest
+
+
 _REAL_STDOUT = None
 
 
@@ -98,14 +153,20 @@ def emit(line):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps (each timed loop runs exactly this many)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--workload", default=None)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cuprof", action="store_true",
                     help="wrap ONE extra device step in cudaProfilerStart/Stop (ncu --profile-from-start off)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs needs --impl native (the reference arm times a CPU sample, not the path's outputs)")
     args.warmup = max(args.warmup, 3) if args.impl == "native" else max(args.warmup, 1)
 
     import bench_workloads as benchlib
@@ -164,6 +225,7 @@ def main():
         sampler.start()
     ms_dev, launches = timed(wl.step_device, args.steps, args.warmup)
     trace(f"device-resident steps timed: {ms_dev / args.steps:.2f} ms/step")
+    dumped = dump_outputs(wl.out, args.dump_outputs) if args.dump_outputs and rank == 0 else None
     if args.cuprof:
         torch.cuda.synchronize()
         torch.cuda.profiler.start()
@@ -201,6 +263,8 @@ def main():
     line.update(wl.extra())
     if tp_obj is not None:
         line["tp"] = tp_obj
+    if dumped is not None:
+        line["dumped_outputs"] = {"dir": os.path.abspath(args.dump_outputs), "arrays": dumped}
     if name == benchlib.DEFAULT_WORKLOAD and not os.environ.get("VLLM_BENCH_NO_EXTRAS"):
         try:                                               # the "deform-attn HBM GB/s" half of BASELINE.json's metric
             line["msda"] = benchlib.msda_extra(torch.device("cuda", local_rank))

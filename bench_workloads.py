@@ -1245,7 +1245,7 @@ def _event_ms(torch, fn, reps, warm=3, flush=None):
 
 def msda_extra(device, reps=20):
     """MSDA forward at the cfg-2b encoder shape on THIS GPU: our kernel (fp32 reference layout = the parity path, and
-    bf16 value = the GDINO modules' path) and, when baseline/_ref/msda holds it, the reference's own CUDA kernel
+    bf16 value = the GDINO modules' path) and, when oracle/_ref/msda holds it, the reference's own CUDA kernel
     recompiled for sm_100.  CUDA events per launch, L2 flushed between launches; GB/s on the algorithmic bytes
     (SURVEY 8d: value + sampling_loc + attn_weight once, output once)."""
     import torch
@@ -1277,7 +1277,7 @@ def msda_extra(device, reps=20):
                             ncu_dram_bytes("r2_msda_win_ncu.json", "msda_fwd_win_kernel<__nv_bfloat16, __nv_bfloat16"))
     try:
         import importlib.util
-        path = os.path.join(ROOT, "baseline", "_ref", "msda", "MultiScaleDeformableAttention.so")
+        path = os.path.join(ROOT, "oracle", "_ref", "msda", "MultiScaleDeformableAttention.so")
         if os.path.exists(path):
             spec = importlib.util.spec_from_file_location("MultiScaleDeformableAttention", path)
             ref = importlib.util.module_from_spec(spec)
@@ -1290,7 +1290,7 @@ def msda_extra(device, reps=20):
             r["max_abs_diff_ours_vs_reference_kernel"] = float((mine - theirs).abs().max())
             out["reference_cuda_kernel_fp32"] = r
         else:
-            out["reference_cuda_kernel_fp32"] = {"unavailable": "baseline/_ref/msda not built (python baseline/build_msda_ref.py)"}
+            out["reference_cuda_kernel_fp32"] = {"unavailable": "oracle/_ref/msda not built (python oracle/build_msda_ref.py, which needs a VisionLLMv2 checkout)"}
     except Exception as e:                                # the reference arm is evidence, never a dependency
         out["reference_cuda_kernel_fp32"] = {"unavailable": f"{type(e).__name__}: {e}"[:200]}
     return out
@@ -1726,15 +1726,14 @@ def run_reference_arm(name, n_gpus, steps, warmup):
     a BOUNDED SAMPLE (one layer of each tower at real width) and the workload figure is EXTRAPOLATED from it -- the
     line says so (`extrapolated`, `sample_ms_per_step`, `steps` = sample steps really run); cfg 1 is measured whole."""
     wl = WORKLOADS[name]
-    run_steps = max(1, min(steps, 20 if name == "cfg1_forward" else 5))
     run_warm = max(1, min(warmup, 2))
     t0 = time.perf_counter()
-    cb = _CPU[name](steps=run_steps, warmup=run_warm)
+    cb = _CPU[name](steps=steps, warmup=run_warm)
     wall = time.perf_counter() - t0
     cb.setdefault("extrapolated", True)
-    cb["steps_run"] = run_steps
+    cb["steps_run"] = steps
     return {"impl": "reference", "metric": wl.metric, "value": cb["value"], "unit": wl.unit, "n_gpus": n_gpus,
-            "steps": run_steps, "steps_requested": steps, "warmup": run_warm, "ms_per_step": cb["ms_per_step"],
+            "steps": steps, "steps_requested": steps, "warmup": run_warm, "ms_per_step": cb["ms_per_step"],
             "extrapolated": cb["extrapolated"], "sample_ms_per_step": cb.get("sample_ms_per_step"), "wall_s": wall,
             "higher_is_better": True,
             "scaling": "strong" if name in ("llm_tp", "llm_tp_plain", "llm_tp_train") else "weak", "vs_baseline": None,

@@ -221,3 +221,19 @@ def test_live_tile_lists_give_the_dense_result(B, H, T, D, group):
     p = torch.softmax(ref_s, -1).nan_to_num(0.0)
     ref = (p @ v.float().permute(0, 2, 1, 3)).permute(0, 2, 1, 3).reshape(B, T, H * D)
     assert ((sparse.float() - ref).norm() / ref.norm()).item() < 6e-3
+
+
+@pytest.mark.parametrize("causal", [True, False])
+def test_attention_is_reproducible_at_the_llm_shape(causal):
+    """The same inputs give bit-identical outputs on every call, at the Vicuna-7B shape of the flagship forward (8 x 1536
+    tokens, 32 heads of 128, q/k/v slices of one packed qkv tensor).  Before the epilogue waited on a barrier committed
+    after the last P V product, tc2 warps could read O from tensor memory early and a few 32-row groups changed between
+    calls."""
+    from visionllm_b200 import ops
+    g = torch.Generator(device="cuda").manual_seed(0)
+    B, T, H, D = 8, 1536, 32, 128
+    qkv = torch.randn(B, T, 3 * H * D, device="cuda", generator=g).bfloat16()
+    q, k, v = (qkv[..., i * H * D:(i + 1) * H * D].unflatten(-1, (H, D)) for i in range(3))
+    first = ops.attention(q, k, v, causal=causal)
+    for _ in range(4):
+        assert torch.equal(ops.attention(q, k, v, causal=causal), first)

@@ -1,106 +1,79 @@
-"""CPU, build container only (needs /root/reference): the drop-in claim of INTEGRATION.md section 4 -- assign the
-B200 layer classes over the reference's names, let the REFERENCE'S OWN `GroundingDinoEncoder` stack (its python
-loop, reference points, hidden-state bookkeeping) drive them, and compare with the untouched reference stack.
-Kernels are replaced by fp32 torch stand-ins here (no GPU in this container); the -m gpu tests cover the kernels."""
+"""CPU: the drop-in claim of INTEGRATION.md section 4 -- the B200 layer classes can stand in for the reference's under
+the REFERENCE'S OWN `GroundingDinoEncoder` / `GroundingDinoDecoder` stacks (their python loops, reference points,
+hidden-state bookkeeping).  tests/golden/gen_golden_gdino_cpu.py ran those stacks and recorded every call they made to
+their layers and heads (keyword arguments and outputs); here the B200 classes, built under the same parameter names with
+the same weights, receive exactly those calls and must return the same outputs.  Kernels are replaced by fp32 torch
+stand-ins here (no GPU in this test); the -m gpu tests cover the kernels."""
+import json
 import os
 import sys
 
-import pytest
+import numpy as np
 import torch
 
-pytestmark = pytest.mark.skipif(not os.path.exists("/root/reference/VisionLLMv2"), reason="reference tree not mounted")
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
 from test_gdino_logic_cpu import torch_kernels  # noqa: E402,F401  (fixture)
+from test_gdino_model_cpu import reference_config  # noqa: E402
 
 
-def test_reference_encoder_stack_runs_on_b200_layers(torch_kernels):  # noqa: F811
-    import ref_shim
-    from weights_util import seeded_state_dict
+def replay(g, modules, tol):
+    """Call modules[name] with every recorded call of the reference module `name`; compare the primary output
+    (encoder layer: (vision, text); decoder layer: hidden states; heads: the tensor) within tol[name]."""
+    def load(e):
+        if "tensor" in e:
+            return torch.from_numpy(g[e["tensor"]])
+        if "seq" in e:
+            return tuple(load(x) for x in e["seq"])
+        return e["value"]
+
+    def tensors(x):
+        return [x] if isinstance(x, torch.Tensor) else [t for y in x for t in tensors(y)]
+
+    calls = json.loads(str(g["calls"]))
+    assert {c["module"] for c in calls} == set(modules)
+    for c in calls:
+        name = c["module"]
+        with torch.no_grad():
+            got = modules[name](*[load(a) for a in c["args"]], **{k: load(v) for k, v in c["kwargs"].items()})
+        want = load(c["output"])
+        if not name.startswith(("bbox_embed", "reference_points_head")):
+            got, want = got[0], want[0]
+        got, want = tensors(got), tensors(want)
+        assert len(got) == len(want), name
+        for a, b in zip(got, want):
+            assert a.shape == b.shape and (a - b).abs().max() < tol(name), name
+
+
+def load_weights(stack, g):
+    from weights_util import key_shapes, seeded_state_dict
+    assert [list(k) for k in key_shapes(stack)] == json.loads(str(g["keys"]))    # identical parameter names
+    stack.load_state_dict(seeded_state_dict(stack, int(g["seed"])), strict=True)
+
+
+def test_reference_encoder_stack_runs_on_b200_layers(golden_dir, torch_kernels):  # noqa: F811
     import visionllm_b200.gdino as b200
-    cfgm, gd = ref_shim.load_gdino()
-    cfg = cfgm.GroundingDinoConfig(d_model=256, encoder_layers=2, encoder_attention_heads=8, encoder_ffn_dim=512,
-                                   num_feature_levels=4, encoder_n_points=4, dropout=0.0, attention_dropout=0.0,
-                                   activation_dropout=0.0, fusion_dropout=0.0, fusion_droppath=0.0,
-                                   text_enhancer_dropout=0.0, disable_custom_kernels=True)
-    ref_enc = gd.GroundingDinoEncoder(cfg).eval()
-    sd = seeded_state_dict(ref_enc, 77)
-    ref_enc.load_state_dict(sd)
-    saved = gd.GroundingDinoEncoderLayer
-    try:
-        gd.GroundingDinoEncoderLayer = b200.GroundingDinoEncoderLayer          # the one-line swap
-        cfg.activation_function = "relu"
-        new_enc = gd.GroundingDinoEncoder(cfg).eval()
-    finally:
-        gd.GroundingDinoEncoderLayer = saved
-    assert type(new_enc.layers[0]).__module__ == "visionllm_b200.gdino"
-    new_enc.load_state_dict(sd, strict=True)                                    # identical parameter names
-    shapes_l = [(8, 10), (4, 5), (2, 3), (1, 2)]
-    shapes = torch.tensor(shapes_l)
-    lsi = torch.cat((shapes.new_zeros(1), shapes.prod(1).cumsum(0)[:-1]))
-    S, B, T = int(shapes.prod(1).sum()), 1, 6
-    g = torch.Generator().manual_seed(1)
-    src, pos, text = (torch.randn(B, S, 256, generator=g), torch.randn(B, S, 256, generator=g) * 0.5,
-                      torch.randn(B, T, 256, generator=g))
-    vmask = torch.zeros(B, S, dtype=torch.bool)
-    tq = torch.ones(B, T, dtype=torch.bool); tq[0, 4:] = False
-    tsa, pids = gd.generate_masks_with_text_query_masks(tq)
-    kw = dict(vision_features=src, vision_attention_mask=vmask, vision_position_embedding=pos, spatial_shapes=shapes,
-              level_start_index=lsi, valid_ratios=torch.ones(B, 4, 2), text_features=text, text_attention_mask=~tq,
-              text_position_embedding=None, text_self_attention_masks=tsa, text_position_ids=pids,
-              output_attentions=False, output_hidden_states=False, return_dict=True)
-    with torch.no_grad():
-        a = ref_enc(**kw)
-        b = new_enc(**kw)
-    assert (a.last_hidden_state_vision - b.last_hidden_state_vision).abs().max() < 1e-4
-    assert (a.last_hidden_state_text - b.last_hidden_state_text).abs().max() < 1e-4
+    g = np.load(os.path.join(golden_dir, "gdino_dropin_enc.npz"))
+    cfg = reference_config(str(g["config"]))
+    stack = torch.nn.Module()
+    stack.layers = torch.nn.ModuleList([b200.GroundingDinoEncoderLayer(cfg) for _ in range(cfg.encoder_layers)])
+    load_weights(stack, g)
+    stack.eval()
+    replay(g, {f"layers.{i}": layer for i, layer in enumerate(stack.layers)}, lambda name: 1e-4)
 
 
-def test_reference_decoder_stack_runs_on_b200_layers(torch_kernels):  # noqa: F811
+def test_reference_decoder_stack_runs_on_b200_layers(golden_dir, torch_kernels):  # noqa: F811
     """The reference's GroundingDinoDecoder (sine box embeddings, query_pos MLP, per-layer box refinement through
     bbox_embed, intermediate stacking) driving B200 decoder layers and B200 MLP heads."""
-    import ref_shim
-    from weights_util import seeded_state_dict
-    import visionllm_b200.gdino as b200
     import visionllm_b200.gdino_heads as b200h
-    cfgm, gd = ref_shim.load_gdino()
-    cfg = cfgm.GroundingDinoConfig(d_model=256, decoder_layers=2, decoder_attention_heads=8, decoder_ffn_dim=512,
-                                   num_feature_levels=4, decoder_n_points=4, dropout=0.0, attention_dropout=0.0,
-                                   activation_dropout=0.0, disable_custom_kernels=True)
-
-    def build():
-        dec = gd.GroundingDinoDecoder(cfg).eval()
-        # OVGroundingDinoForObjectDetection shares one bbox head per layer with the decoder (gd.py:2640-2652)
-        dec.bbox_embed = torch.nn.ModuleList([gd.GroundingDinoMLPPredictionHead(256, 256, 4, 3) for _ in range(2)])
-        return dec
-
-    ref_dec = build()
-    sd = seeded_state_dict(ref_dec, 88)
-    ref_dec.load_state_dict(sd)
-    saved = (gd.GroundingDinoDecoderLayer, gd.GroundingDinoMLPPredictionHead)
-    try:
-        gd.GroundingDinoDecoderLayer = b200.GroundingDinoDecoderLayer
-        gd.GroundingDinoMLPPredictionHead = b200h.GroundingDinoMLPPredictionHead
-        cfg.activation_function = "relu"
-        new_dec = build()
-    finally:
-        gd.GroundingDinoDecoderLayer, gd.GroundingDinoMLPPredictionHead = saved
-    assert type(new_dec.layers[0]).__module__ == "visionllm_b200.gdino"
-    assert type(new_dec.reference_points_head).__module__ == "visionllm_b200.gdino_heads"
-    new_dec.load_state_dict(sd, strict=True)
-    shapes_l = [(8, 10), (4, 5), (2, 3), (1, 2)]
-    shapes = torch.tensor(shapes_l)
-    lsi = torch.cat((shapes.new_zeros(1), shapes.prod(1).cumsum(0)[:-1]))
-    S, B, Q, T = int(shapes.prod(1).sum()), 2, 9, 5
-    g = torch.Generator().manual_seed(2)
-    kw = dict(inputs_embeds=torch.randn(B, Q, 256, generator=g), vision_encoder_hidden_states=torch.randn(B, S, 256, generator=g),
-              mask_features=None, vision_encoder_attention_mask=torch.ones(B, S, dtype=torch.bool),
-              text_encoder_hidden_states=torch.randn(B, T, 256, generator=g),
-              text_encoder_attention_mask=torch.tensor([[False] * 5, [False, False, False, True, True]]),
-              reference_points=torch.rand(B, Q, 4, generator=g) * 0.5 + 0.2, spatial_shapes=shapes,
-              level_start_index=lsi, valid_ratios=torch.ones(B, 4, 2), self_attn_mask=None, output_attentions=False,
-              output_hidden_states=False, return_dict=True)
-    with torch.no_grad():
-        a = ref_dec(**kw)
-        b = new_dec(**kw)
-    assert (a.intermediate_hidden_states - b.intermediate_hidden_states).abs().max() < 1e-4
-    assert (a.intermediate_reference_points - b.intermediate_reference_points).abs().max() < 1e-5
+    from visionllm_b200.gdino_model import _Decoder
+    g = np.load(os.path.join(golden_dir, "gdino_dropin_dec.npz"))
+    cfg = reference_config(str(g["config"]))
+    dec = _Decoder(cfg)
+    dec.bbox_embed = torch.nn.ModuleList([b200h.GroundingDinoMLPPredictionHead(256, 256, 4, 3)
+                                          for _ in range(cfg.decoder_layers)])
+    load_weights(dec, g)
+    dec.eval()
+    modules = {"reference_points_head": dec.reference_points_head}
+    for i in range(cfg.decoder_layers):
+        modules[f"layers.{i}"], modules[f"bbox_embed.{i}"] = dec.layers[i], dec.bbox_embed[i]
+    replay(g, modules, lambda name: 1e-5 if name.startswith("bbox_embed") else 1e-4)

@@ -1,5 +1,5 @@
-"""The reference's own MSDA CUDA kernel (baseline/_ref/msda, built by baseline/build_msda_ref.py from the sources
-under /root/reference, recompiled for sm_100) timed beside ours on the same B200 at the BASELINE cfg 2b shapes, plus a
+"""The reference's own MSDA CUDA kernel (oracle/_ref/msda, built by oracle/build_msda_ref.py from the reference's
+sources, recompiled for sm_100) timed beside ours on the same B200 at the BASELINE cfg 2b shapes, plus a
 GPU-side parity check against it (SURVEY 8c row 2: "the kernel to beat").
 
     python tools/msda_ref_bench.py [--out profiles/r2_msda_vs_reference_kernel.json]
@@ -16,7 +16,7 @@ sys.path.insert(0, ROOT)
 
 def load_reference_ext():
     import torch  # noqa: F401  (libtorch must be loaded first)
-    path = os.path.join(ROOT, "baseline", "_ref", "msda", "MultiScaleDeformableAttention.so")
+    path = os.path.join(ROOT, "oracle", "_ref", "msda", "MultiScaleDeformableAttention.so")
     if not os.path.exists(path):
         return None
     spec = importlib.util.spec_from_file_location("MultiScaleDeformableAttention", path)

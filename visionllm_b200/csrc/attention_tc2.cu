@@ -137,6 +137,9 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_const
   auto p_ready = [&](int b) { return bar + 8 * (11 + b); };
   const uint32_t o_full = bar + 8 * 13;
   const uint32_t tmem_slot = bar + 8 * 14;
+  // committed once, after the last PV: the epilogue cannot wait on o_full's parity, because when the softmax finishes
+  // its last tile only PV(n-3) is known to have landed and o_full may still be two phases behind
+  const uint32_t o_done = bar + 8 * 15;
   uint32_t* tmem_slot_gen = reinterpret_cast<uint32_t*>(gen + (tmem_slot - base));
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -160,6 +163,7 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_const
       tc::mbar_init(s_full(s), 1); tc::mbar_init(p_ready(s), 128);
     }
     tc::mbar_init(o_full, 1);
+    tc::mbar_init(o_done, 1);
     tc::mbar_fence_init();
   }
   if (warp == 2) tc::tmem_alloc<1>(tmem_slot, TMEM_COLS);
@@ -232,6 +236,8 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_const
           __syncwarp();
         }
       }
+      if (tc::elect_one()) tc::umma_commit<1>(o_done);
+      __syncwarp();
     }
   } else if (warp >= 4) {
     // ===================== softmax warpgroup: one thread per query row =====================
@@ -320,7 +326,7 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_const
     }
     // epilogue: O / l -> bf16, 32 columns at a time
     if (n > 0) {
-      tc::mbar_wait(o_full, (n - 1) & 1);
+      tc::mbar_wait(o_done, 0);
       tc::tc_fence_after();
     }
     if (a.n_splits > 1) {
